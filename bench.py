@@ -2,13 +2,17 @@
 """bench.py -- view-tuples/sec of the hot path on synthetic 5-view x 1024-keypoint tuples.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg3|cfg2|cfg4|cfg5] [--tuples B]
+                    [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of B synthetic units per GPU.  Default = BASELINE.json
 configs[2] (cfg3: ScanNet-shape 5-tuple, 1024 kpts, 28-layer matcher, confidence head, 10 x {w8pt + two-view BA},
 spanning tree, rotation averaging + LUD, global LM BA); --config cfg2 / cfg4 are the two-view workloads
 (configs[1] / [3]: pairs/sec at 1024 / 2048 kpts, w8pt_ba).  One JSON line on rank 0; see DESIGN.md §measurement
-for every field.  `--impl reference` times the CPU port of the reference path (oracle/) on the host cores --
-/root/reference does not exist on the GPU box.
+for every field.  `--impl reference` times the CPU port of the reference path (oracle/) on the host cores; the
+reference project itself is not needed.
+
+`--dump-outputs DIR` writes what the last timed step of rank 0 returned (see dump_outputs) as DIR/<name>.npy.  Weights
+and inputs are seeded, so two builds of the project run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -100,6 +104,35 @@ def emit(line):
     sys.stdout.flush()
     sys.stdout.write('\n' + json.dumps(line) + '\n')
     sys.stdout.flush()
+
+
+DUMP_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """--dump-outputs: every numeric array of `arrays` (torch tensors or numpy) as <out_dir>/<name>.npy, float64 for
+    float64 and integer results, float32 for the rest (both exact).  To stay within `budget` bytes in all, an array
+    of more than `cap` elements is replaced by its elements at `cap` fixed positions (flat, C order, increasing),
+    drawn from a seeded generator: runs with the same arguments dump the same positions.  `cap` is the largest
+    halving of the biggest array's size that fits the budget.  -> {name: stored element count}."""
+    import torch
+    host = {}
+    for name, v in arrays.items():
+        if isinstance(v, torch.Tensor):
+            v = v.detach().cpu().numpy()
+        if isinstance(v, np.ndarray) and v.dtype.kind in 'biuf':
+            host[name] = v.astype(np.float64 if v.dtype.kind in 'iu' or v.dtype == np.float64 else np.float32)
+    cap = max([v.size for v in host.values()] + [1])
+    while cap > 1 and sum(min(v.size, cap) * v.itemsize for v in host.values()) > budget:
+        cap //= 2
+    os.makedirs(out_dir, exist_ok=True)
+    stored = {}
+    for name, v in host.items():
+        if v.size > cap:
+            v = v.reshape(-1)[np.sort(np.random.default_rng(0).choice(v.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name + '.npy'), v)
+        stored[name] = v.size
+    return stored
 
 
 def load_traffic(workload, batch):
@@ -380,9 +413,11 @@ def run_train_arm(args, cfg, rank, world, local):
     data_dev = dict({k: v.to(dev) for k, v in host.items()}, **fixed)
     h2d_bytes = sum(v.numel() * v.element_size() for v in host.values())
     loss_host = torch.zeros(1).pin_memory()
+    last = {}
 
     def step_device():
-        return training.train_step(opt, dict(data_dev), model, optimizer, P)[0]
+        last['loss'], last['losses'] = training.train_step(opt, dict(data_dev), model, optimizer, P)
+        return last['loss']
 
     def step_e2e():
         d = dict({k: v.to(dev, non_blocking=True) for k, v in host.items()}, **fixed)
@@ -416,6 +451,12 @@ def run_train_arm(args, cfg, rank, world, local):
     n0 = lib.mvm_launch_count()
     ms_dev = timed(step_device, args.steps)
     launches = lib.mvm_launch_count() - n0
+    if args.dump_outputs and rank == 0:
+        # a training step returns its losses and leaves the gradients and the updated weights in the model
+        named = list(model.named_parameters())
+        dump_outputs(args.dump_outputs, dict(last['losses'], loss=last['loss'],
+                                             **{'grad.' + k: p.grad for k, p in named if p.grad is not None},
+                                             **{'param.' + k: p for k, p in named}))
     ms_e2e = timed(step_e2e, args.steps)
     sampler.stop_flag = True
     losses.append(float(step_device()))
@@ -505,7 +546,12 @@ def main():
                     help='operand planes of the mode-3 layer GEMMs (persistent kernel): 0 = tf32 hi/lo, 1 = fp16 hi/lo')
     ap.add_argument('--math-mode', type=int, default=3, choices=[0, 1, 3],
                     help='3 = tcgen05 3xTF32 (fp32-faithful, default), 1 = tcgen05 single-pass TF32, 0 = fp32 CUDA cores')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the arrays the last timed step returned as DIR/<name>.npy (float32 / float64, '
+                         'at most 64 MB in all: larger outputs are stored as a fixed, seeded sample)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs records the outputs of --impl ours')
     cfg = CONFIGS[args.config]
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
     rank = int(os.environ.get('RANK', 0))
@@ -574,7 +620,7 @@ def main():
 
     def step_device():
         res, pose = pipe(data_dev)
-        last['res'] = res
+        last['res'], last['pose'] = res, pose
         if world > 1:   # the per-rank loss is accumulated on the device; ONE all-reduce closes the timed region
             loss.add_(step_loss(pose))
         return pose
@@ -661,6 +707,9 @@ def main():
     n0 = lib.mvm_launch_count()
     ms_dev, wall_dev = timed(step_device, args.steps)
     launches = lib.mvm_launch_count() - n0
+    if args.dump_outputs and rank == 0:
+        # pose is None when fewer than two views have keypoints (pipeline.py); its arrays carry a 'pose.' prefix
+        dump_outputs(args.dump_outputs, dict(last['res'], **{'pose.' + k: v for k, v in (last['pose'] or {}).items()}))
     staged.clear()                 # the first timed step stages its own inputs inside the timed region
     ms_e2e, wall_e2e = timed(step_e2e, args.steps)
     e2e_steps = [round(x, 2) for x in last['per_step_ms']]

@@ -100,7 +100,8 @@ def main():
             small['norm__' + k] = np.float64(np.linalg.norm(g64))
             rel[k] = float(small['noise__' + k] / max(np.abs(g64).max(), 1e-30))
         for k in [k[len('f64__inter__'):] for k in out if k.startswith('f64__inter__')]:
-            small['inter__' + k] = out['f64__inter__' + k].astype(np.float32)
+            flat = out['f64__inter__' + k].reshape(-1)
+            small['inter__' + k] = flat[sample_index('inter__' + k, flat.size)].astype(np.float32)
             small['inter_noise__' + k] = np.float64(np.abs(out['f32__inter__' + k].astype(np.float64) - out['f64__inter__' + k]).max())
         worst = max(rel, key=rel.get)
         report[case['name']] = {'loss_f64': float(out['f64__loss']), 'loss_f32': float(out['f32__loss']), 'n_params_with_grad': len(names),

@@ -47,17 +47,7 @@ def main():
             model = model.to(dtype).train()
             data = {k: (torch.from_numpy(v).to(dtype) if isinstance(v, np.ndarray) and v.dtype.kind == 'f' else v)
                     for k, v in data_np.items()}
-            inter = {}
-            hooks = []
-            if case['multi']:       # intermediates of the stacked train branch ([T, B, 256, N]) for stage-level diagnosis
-                hooks.append(model.kenc.register_forward_hook(lambda m, i, o: inter.__setitem__('kenc', o.detach().numpy())))
-                hooks.append(model.gnn.register_forward_hook(lambda m, i, o: inter.__setitem__('gnn', o.detach().numpy())))
-                hooks.append(model.gnn.layers[0].register_forward_hook(lambda m, i, o: inter.__setitem__('layer0_delta', o.detach().numpy())))
             res = model(data)
-            for h_ in hooks:
-                h_.remove()
-            for k, v in inter.items():
-                out['%s__inter__%s' % (tag, k)] = v
             st = model.state_dict()
             for k, v in res.items():
                 if v is not None:

@@ -84,4 +84,29 @@ def test_pair_config_lines():
 
 def test_bench_cli_parses_without_gpu():
     r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--help'], capture_output=True, text=True, timeout=120)
-    assert r.returncode == 0 and '--impl' in r.stdout and '--gpus' in r.stdout
+    assert r.returncode == 0 and '--impl' in r.stdout and '--gpus' in r.stdout and '--dump-outputs' in r.stdout
+
+
+def test_dump_outputs_exact_small_sampled_large(tmp_path):
+    """bench.py --dump-outputs: small outputs stored exactly as float32 / float64, a large one as a seeded sample that
+    keeps the total within the budget, the same positions on every run."""
+    import numpy as np
+    import torch
+    import bench
+    big = np.arange(1 << 16, dtype=np.float32).reshape(64, 1024)
+    arrays = {'scores': torch.from_numpy(big), 'matches': torch.arange(-1, 99), 'success': torch.tensor([True, False]),
+              'cost': np.linspace(0.0, 1.0, 7), 'view_ids': [0, 1]}
+    budget = 1 << 16
+    stored = bench.dump_outputs(str(tmp_path / 'a'), arrays, budget=budget)
+    bench.dump_outputs(str(tmp_path / 'b'), arrays, budget=budget)
+    assert sorted(stored) == ['cost', 'matches', 'scores', 'success']
+    assert sorted(os.listdir(tmp_path / 'a')) == sorted(n + '.npy' for n in stored)
+    a = {n: np.load(tmp_path / 'a' / (n + '.npy')) for n in stored}
+    assert sum(v.nbytes for v in a.values()) <= budget
+    assert a['matches'].dtype == np.float64 and np.array_equal(a['matches'], np.arange(-1, 99))
+    assert a['success'].dtype == np.float32 and a['success'].tolist() == [1.0, 0.0]
+    assert a['cost'].dtype == np.float64 and np.array_equal(a['cost'], arrays['cost'])
+    s = a['scores']                      # element k of `big` is k: the sample holds its own (increasing) positions
+    assert s.dtype == np.float32 and 0 < s.size < big.size and np.all(np.diff(s) > 0)
+    for n in stored:
+        assert np.array_equal(a[n], np.load(tmp_path / 'b' / (n + '.npy')))

@@ -1,7 +1,7 @@
 """Full-size parity at the BASELINE.json configurations: the CUDA matcher against fixtures produced by the
 UNMODIFIED reference at 5 x 1024 kpts x 28 layers (cfg3, the bench workload), 2 x 1024 x 18 layers (cfg2, batch 2)
 and 2 x 2048 x 18 layers (cfg4) -- oracle/make_golden_full.py.  Per pair the fixture holds the matches, matching
-scores and confidences in full, 25 rows of the coupling matrix and float64 checksums of the whole matrix, plus
+scores and confidences in full, 25 rows of the coupling matrix (9 for cfg3) and float64 checksums of the whole matrix, plus
 the same rows from the reference's own double-precision run, whose distance to the fp32 run (`noise`) is the
 yardstick for the score tolerance."""
 import json

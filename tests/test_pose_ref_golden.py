@@ -55,8 +55,6 @@ def test_w8pt_choose_closest_oracle_vs_reference_golden():
 def test_ba2view_oracle_vs_reference_golden(path):
     from oracle import pose as P
     z = np.load(path)
-    if z['kpts0_norm'].shape[1] > 600:
-        pytest.skip('dense (6+3n)^2 oracle at n = 1024 takes minutes; checked by the generator')
     ext, valid = P.run_bundle_adjust_2_view(z['kpts0_norm'].astype(np.float64), z['kpts1_norm'].astype(np.float64),
                                             z['conf'].astype(np.float64), z['T_init'].astype(np.float64), 10)
     assert np.array_equal(valid, z['valid64']) and np.array_equal(valid, z['valid32'])

@@ -5,14 +5,15 @@ sign, its ReLU mask flips, and the gradient w.r.t. the MLP hidden layer (g_hid) 
 that element -- orders of magnitude above rounding -- which reaches the keypoint-encoder gradient as 3e-3 .. 7e-3.
 Output committed as profiles/r02_train_kink.txt."""
 import sys, json, os, numpy as np, torch
-sys.path.insert(0,'/root/repo')
+ROOT=os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0,ROOT)
 import tools.train_diag as Dg
 from tests import emul_ops
 from e2e_multi_view_matching_b200 import ops,_lib
 for f in Dg.PATCHED: setattr(ops,f,getattr(emul_ops,f))
 _lib.require_cuda=lambda d,w:None
 name='mv3_64'
-z=np.load('/root/repo/tests/golden/train_backward_%s.npz'%name); case=json.loads(str(z['meta']))
+z=np.load(os.path.join(ROOT,'tests','golden','train_backward_%s.npz'%name)); case=json.loads(str(z['meta']))
 data_np,sd=Dg.build(case)
 f64,b64,r64,l64=Dg.run(case,sd,data_np,'cpu')
 base_lin=emul_ops.linear
